@@ -1,13 +1,15 @@
 #!/usr/bin/env python
 """bench.py — E4T pre-training throughput on B200 (BASELINE.json metric: images/sec @512², per-GPU bs16, SD-v1.4).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 16] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--batch 16] [--impl ours|reference] [--dump-outputs DIR]
 
 One "step" = one pass of the hot path (pretrain_e4t.py:595-654: UNet encoder-half -> E4T encoder -> text encoder ->
 full UNet -> loss -> backward -> AdamW) over one batch of synthetic 512² inputs with random-init SD-v1.4 + ViT-H/14
 weights.  Prints ONE JSON line (rank 0).  `value` = device-resident throughput (inputs already in HBM), `e2e` = the
 same through the public API with pinned-host inputs copied every step and the loss read back every step.
 `--impl reference` times the CPU oracle (oracle/e4t_oracle.py, the restated reference path) on the host cores.
+`--dump-outputs DIR` writes what the last timed step produced as DIR/<name>.npy (float32), so that two builds run with
+the same arguments (hence the same seeded weights and inputs) can be compared output for output.
 """
 import argparse
 import json
@@ -38,6 +40,9 @@ def parse():
     ap.add_argument("--impl", default="ours", choices=["ours", "reference", "torch_stock"],
                     help="reference = the reference's CPU path on the host cores; torch_stock = the same step in stock torch "
                          "ops (cuBLAS/cuDNN/SDPA, bf16 autocast) on the GPU: the on-box library comparator")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the last step's losses and a fixed sample of the updated trainable "
+                         "parameters and AdamW first moments as DIR/<name>.npy")
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--no-micro", action="store_true")
@@ -152,6 +157,22 @@ def host_batch(B, seed, pinned=True):
     if pinned:
         b = {k: v.pin_memory() for k, v in b.items()}
     return b
+
+
+DUMP_SAMPLE = 1 << 22      # entries of each sampled optimiser buffer: 2 x 16 MB of float32
+
+
+def dump_outputs(dirname, out, opt):
+    """The step's loss terms as returned to the caller, and the same seeded sample of the flat parameter arena and of
+    AdamW's first moment (the latter carries the gradients, which the sign-like early AdamW update mostly hides)."""
+    import numpy as np
+    os.makedirs(dirname, exist_ok=True)
+    idx = torch.randint(0, opt.arena.numel(), (min(DUMP_SAMPLE, opt.arena.numel()),),
+                        generator=torch.Generator().manual_seed(0)).to(opt.arena.device)
+    arrays = {k: v.detach().float() for k, v in out.items() if torch.is_tensor(v) and v.is_floating_point()}
+    arrays.update(params_sample=opt.arena[idx], exp_avg_sample=opt.exp_avg[idx])
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, f"{k}.npy"), v.cpu().numpy().astype(np.float32))
 
 
 def to_device(b, device):
@@ -456,11 +477,11 @@ def main():
         torch.cuda.synchronize()
 
     def run_steps(n, batches, e2e):
-        """n steps; returns device time (s) via CUDA events and the last loss."""
+        """n steps; returns device time (s) via CUDA events, the last loss and the last step's outputs."""
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         barrier()
         e0.record()
-        last = None
+        last = out = None
         for i in range(n):
             hb = batches[i % len(batches)]
             # e2e: pinned host -> device every step (straight into the graph's static inputs when graphed)
@@ -477,7 +498,7 @@ def main():
             tt = torch.tensor([t], device=device)
             dist.all_reduce(tt, op=dist.ReduceOp.MAX)
             t = tt.item()
-        return t, (last if isinstance(last, float) else float(last))
+        return t, (last if isinstance(last, float) else float(last)), out
 
     host_batches = [host_batch(B, 42 + rank * 1000 + i) for i in range(4)]
     if args.tuning:      # one image (and its latents) repeated over the batch, fresh noise / timesteps per step (:266-281)
@@ -506,8 +527,11 @@ def main():
     if rank == 0:
         sampler.start()
     _lib.reset_launch_count()
-    t_dev, loss = run_steps(args.steps, dev_batches, False)
+    t_dev, loss, out = run_steps(args.steps, dev_batches, False)
     launches = _lib.launch_count()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, out, step.opt)
+    del out
     if cuda_graph is True:
         # under graph replay the host-side counter does not tick: count the launches of one eager step instead
         step_graph, step._graph = step._graph, None
@@ -521,7 +545,7 @@ def main():
     e2e = None
     if not args.no_e2e:
         run_steps(1, host_batches, True)
-        t_e2e, _ = run_steps(args.steps, host_batches, True)
+        t_e2e, _, _ = run_steps(args.steps, host_batches, True)
         e2e = {"value": world * B * args.steps / t_e2e, "unit": "images/sec", "h2d_bytes_per_step": h2d,
                "d2h_bytes_per_step": 4, "ms_per_step": t_e2e / args.steps * 1e3}
 

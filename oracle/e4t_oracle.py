@@ -9,8 +9,8 @@ the reference's exact key names.  Each function cites the reference file:line it
 
 Pinning status
   * UNet + WeightOffsets + attention + transformer blocks: PINNED — oracle/gen_golden.py imports the reference's own
-    e4t/models/*.py from /root/reference (through oracle/shim for the absent diffusers package) and the outputs /
-    gradients it produced are committed under tests/golden/ (tests/test_oracle_cpu.py checks this file against them).
+    e4t/models/*.py from a checkout of the original project (through oracle/shim for the absent diffusers package) and
+    the outputs / gradients it produced are committed under tests/golden/ (tests/test_oracle_cpu.py checks this file against them).
   * diffusers 0.14.0 pieces (ResnetBlock2D, Downsample2D, Upsample2D, Timesteps, TimestepEmbedding, DDPM add_noise):
     restated from the published 0.14.0 behaviour — **parity unpinned** (diffusers is not installed, no network).
   * E4TEncoder (e4t/encoder.py:78-168): open_clip and kornia are absent, so the ViT-H/14 tower follows open_clip's

@@ -1,7 +1,7 @@
-"""Generate tests/golden/*.pt by running the REFERENCE's own modules (imported unchanged from /root/reference via
-oracle/shim) on seeded synthetic weights/inputs.  Run in the build container only (the GPU box has no /root/reference):
+"""Generate tests/golden/*.pt by running the REFERENCE's own modules (imported unchanged from a checkout of the original
+e4t-diffusion project via oracle/shim) on seeded synthetic weights/inputs:
 
-    python oracle/gen_golden.py            # writes tests/golden/{unet_tiny,unet_sd14,wo,inventory}.pt
+    E4T_REFERENCE=<checkout> python oracle/gen_golden.py    # writes tests/golden/{unet_tiny,unet_sd14,wo,inventory}.pt
 
 The fixtures pin oracle/e4t_oracle.py (tests/test_oracle_cpu.py) and are the parity target of the CUDA path
 (tests/test_e2e_gpu.py).  Everything is fp32 on CPU; weights come from e4t_oracle.synth_state_dict so the oracle and
@@ -16,9 +16,12 @@ import torch
 
 HERE = os.path.dirname(os.path.abspath(__file__))
 ROOT = os.path.dirname(HERE)
-sys.path[:0] = ["/root/reference", os.path.join(HERE, "shim"), ROOT]
+if not os.path.isdir(os.environ.get("E4T_REFERENCE", "")):
+    raise SystemExit("set E4T_REFERENCE to a checkout of the original e4t-diffusion project")
+sys.path[:0] = [os.environ["E4T_REFERENCE"], os.path.join(HERE, "shim"), ROOT]
 
 from oracle import e4t_oracle as O  # noqa: E402
+from oracle.golden import sample_grads, sample_rows  # noqa: E402
 
 from e4t.models.unet_2d_condition import UNet2DConditionModel  # noqa: E402  (the reference's)
 from e4t.weightoffsets import WeightOffsets  # noqa: E402
@@ -77,7 +80,7 @@ def wo_case():
         mod = WeightOffsets(R, C)
         sd = O.synth_state_dict({("p." + k): tuple(v.shape) for k, v in mod.state_dict().items()}, 3)
         mod.load_state_dict({k[2:]: v for k, v in sd.items()})
-        rec[(R, C)] = mod().detach().clone()
+        rec[(R, C)] = sample_rows(mod().detach(), 1 if R * C <= 320 * 320 else 4)
     return rec
 
 
@@ -87,7 +90,9 @@ def main():
     print("tiny unet"); torch.save(unet_case(O.TINY_UNET, 2, 1, True, 16), os.path.join(OUT, "unet_tiny.pt"))
     print("sd14 unet")
     rec = unet_case(O.SD14_UNET, 1, 2, True, 64)
-    # keep the big fixture small: drop the corner copies of 1280^2 matrices? they are 16x16 already.
+    # below 1 MB: the tests re-draw `w` from the seed, and keep a fixed sample of the WeightOffsets gradients
+    del rec["w"]
+    rec["wo_grads"] = sample_grads(rec["wo_grads"], 16)
     torch.save(rec, os.path.join(OUT, "unet_sd14.pt"))
     m = UNet2DConditionModel(**O.ref_unet_kwargs(O.SD14_UNET))
     keys = sorted(m.state_dict().keys())

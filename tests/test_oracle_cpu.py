@@ -1,5 +1,5 @@
 """Pin the CPU oracle (oracle/e4t_oracle.py) against the golden vectors produced by the REFERENCE's own modules
-(oracle/gen_golden.py, run in the build container with /root/reference importable).  fp32, tolerance 1e-4 relative
+(oracle/gen_golden.py, run with a checkout of the original project importable).  fp32, tolerance 1e-4 relative
 (summation-order differences only)."""
 import os
 
@@ -21,10 +21,11 @@ def test_wo_literal_and_closed_form_match_reference():
     for (R, C), ref in gold.items():
         shapes = O._wo_shapes("p.", R, C)
         sd = O.synth_state_dict(shapes, 3)
-        assert _rel(O.wo_delta(sd, "p."), ref) < 1e-5
+        got = O.wo_delta(sd, "p.")
+        assert got.shape == (C, R)
+        assert _rel(got[::ref["row_stride"]], ref["rows"]) < 1e-5
         sd64 = {k: v.double() for k, v in sd.items()}
         assert _rel(O.wo_delta_closed_form(sd64, "p."), O.wo_delta(sd64, "p.")) < 1e-12
-        assert ref.shape == (C, R)
 
 
 def test_inventory_matches_reference_state_dict():
