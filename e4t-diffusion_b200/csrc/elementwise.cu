@@ -460,6 +460,35 @@ extern "C" int e4t_conv_in_fwd(const float* x, const float* w, const float* bias
   return 0;
 }
 
+// 1x1 convolution on NCHW fp32, y[b][o][p] = bias[o] + sum_i w[o][i] x[b][i][p] (Cin, Cout <= 8): the VAE's
+// post_quant_conv on the latents, applied on its own so that the decoder's conv_in zero-pads the transformed latents.
+__global__ void pointwise_nchw_kernel(const float* __restrict__ x, const float* __restrict__ w,
+                                      const float* __restrict__ bias, float* __restrict__ y, int B, int Cin, int Cout,
+                                      long HW) {
+  for (long i = (long)blockIdx.x * blockDim.x + threadIdx.x; i < (long)B * HW; i += (long)gridDim.x * blockDim.x) {
+    const long b = i / HW, p = i % HW;
+    float xv[8];
+#pragma unroll
+    for (int c = 0; c < 8; ++c) xv[c] = c < Cin ? x[(b * Cin + c) * HW + p] : 0.f;
+    for (int o = 0; o < Cout; ++o) {
+      float acc = bias ? bias[o] : 0.f;
+#pragma unroll
+      for (int c = 0; c < 8; ++c)
+        if (c < Cin) acc = fmaf(w[o * Cin + c], xv[c], acc);
+      y[(b * Cout + o) * HW + p] = acc;
+    }
+  }
+}
+extern "C" int e4t_pointwise_nchw(const float* x, const float* w, const float* bias, float* y, int B, int Cin, int Cout,
+                                  long long HW, void* stream_) {
+  E4T_CHECK(Cin >= 1 && Cin <= 8 && Cout >= 1 && Cout <= 8, "e4t_pointwise_nchw: Cin, Cout must be in [1, 8]");
+  pointwise_nchw_kernel<<<grid_for((long)B * HW, 256), 256, 0, (cudaStream_t)stream_>>>(x, w, bias, y, B, Cin, Cout,
+                                                                                       (long)HW);
+  E4T_COUNT_LAUNCH();
+  E4T_LAUNCH_CHECK();
+  return 0;
+}
+
 // conv_out: NHWC bf16 (B,H,W,C) -> NCHW fp32 (B,Cout<=8,H,W); w fp32 [Cout][C][3][3].  One warp per pixel.
 __global__ void conv_out_fwd_kernel(const bf16* __restrict__ x, const float* __restrict__ w,
                                     const float* __restrict__ bias, float* __restrict__ y, int B, int H, int W, int C,

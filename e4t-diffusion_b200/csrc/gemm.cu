@@ -23,6 +23,7 @@ struct GemmArgs {
   // implicit 3x3 convolution (conv = 1: forward / dgrad, 2: weight gradient)
   int conv, H, W, BH, BB, cin_chunks, cout;
   int cstride;   // spatial stride of the forward convolution (1, or 2 = Downsample2D; H, W are the OUTPUT size)
+  int cpad;      // top/left zero padding of the forward convolution (1, or 0 = the VAE's F.pad(x, (0,1,0,1)) downsample)
   // epilogue
   void* out;
   int out_mode;  // 0 = bf16 store, 1 = fp32 store, 2 = fp32 atomic add
@@ -101,11 +102,14 @@ e4t_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
         const int m0 = m_t * kBM, n0 = n_t * g.BN;
         const int kc0 = sp * g.kper;
         const int kc1 = min(g.kchunks, kc0 + g.kper);
-        int cb0 = 0, ch0 = 0;
+        // first output pixel of the tile: image cb0, row ch0, column cw0 (cw0 > 0 only for images wider than 128,
+        // where a tile is a 128-pixel segment of one row)
+        int cb0 = 0, ch0 = 0, cw0 = 0;
         if (g.conv == 1) {
           const int img = g.H * g.W;
           cb0 = m0 / img;
           ch0 = (m0 % img) / g.W;
+          cw0 = m0 % g.W;
         }
         for (int kc = kc0; kc < kc1; ++kc) {
           mbar_wait(&empty_bar[s], ph ^ 1u);
@@ -130,7 +134,8 @@ e4t_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
           } else if (g.conv) {
             const int tap = kc / g.cin_chunks, cc = kc % g.cin_chunks;
             const int dy = tap / 3, dx = tap % 3;
-            tma_load_4d(sA, &mapA, &full_bar[s], cc * kBK, dx - 1, g.cstride * ch0 + dy - 1, cb0);
+            tma_load_4d(sA, &mapA, &full_bar[s], cc * kBK, g.cstride * cw0 + dx - g.cpad, g.cstride * ch0 + dy - g.cpad,
+                        cb0);
             tma_load_2d(sB, &mapB, &full_bar[s], cc * kBK, tap * g.cout + n0);
           } else {
             const int ab = g.a_batched ? bz : 0, bb = g.b_batched ? bz : 0;
@@ -674,17 +679,26 @@ extern "C" int e4t_gemm_bf16(const void* A, const void* B, void* out, int M, int
 // stride 2 (diffusers Downsample2D): the A-operand tensor map walks the input with element strides (1,2,2,1), so the
 // tile of 128 OUTPUT pixels is gathered directly from every other input pixel — no stride-1 result is computed and
 // thrown away (round 1 did exactly that: 4x the FLOPs on the three downsampling convolutions).
+// Output widths above 128 (the VAE at 256 and 512 pixels) must be multiples of 128: each 128-row M tile is then a
+// 128-pixel segment of one image row, and the producer offsets the A-operand box by the segment's first column.
+// pad 0 (stride 2 only): diffusers' VAE Downsample2D, F.pad(x, (0,1,0,1)) then a pad-0 conv; the bottom/right zero
+// row and column come from the TMA out-of-bounds fill.
 static int conv3x3_impl(const void* x, const void* w, void* out, int B, int Hin, int Win, int Cin, int Cout, int stride,
-                        int out_mode, const float* bias, const float* rowgroup, const void* residual, int force_bn,
-                        cudaStream_t stream) {
+                        int pad, int out_mode, const float* bias, const float* rowgroup, const void* residual,
+                        int force_bn, cudaStream_t stream) {
   E4T_CHECK(Cin % 64 == 0, "e4t_conv3x3: Cin must be a multiple of 64 (got %d)", Cin);
   E4T_CHECK(stride == 1 || (stride == 2 && Hin % 2 == 0 && Win % 2 == 0), "e4t_conv3x3: bad stride/size");
+  E4T_CHECK(pad == 1 || (pad == 0 && stride == 2), "e4t_conv3x3: pad must be 1, or 0 with stride 2 (got %d)", pad);
   const int H = Hin / stride, W = Win / stride;
-  E4T_CHECK(W <= 128 && (128 % W) == 0, "e4t_conv3x3: output width must divide 128 (got %d)", W);
+  E4T_CHECK((W <= 128 && (128 % W) == 0) || (W % 128) == 0,
+            "e4t_conv3x3: output width must divide 128 or be a multiple of 128 (got %d)", W);
   E4T_CHECK(out_mode == 0 || out_mode == 1, "e4t_conv3x3: bad out_mode");
   const int img = H * W;
   int BH, BB;
-  if (img >= 128) {
+  if (W >= 128) {
+    BB = 1;
+    BH = 1;
+  } else if (img >= 128) {
     BB = 1;
     BH = 128 / W;
     E4T_CHECK(H % BH == 0, "e4t_conv3x3: H=%d not a multiple of tile height %d", H, BH);
@@ -697,6 +711,7 @@ static int conv3x3_impl(const void* x, const void* w, void* out, int B, int Hin,
   memset(&g, 0, sizeof(g));
   g.M = B * img; g.N = Cout; g.K = Cin; g.batch = 1;
   g.conv = 1; g.H = H; g.W = W; g.BH = BH; g.BB = BB; g.cin_chunks = Cin / 64; g.cout = Cout; g.cstride = stride;
+  g.cpad = pad;
   g.m_tiles = cdiv(g.M, kBM);
   g.kchunks = 9 * g.cin_chunks;
   g.kper = g.kchunks; g.splits = 1;
@@ -710,7 +725,8 @@ static int conv3x3_impl(const void* x, const void* w, void* out, int B, int Hin,
   {
     uint64_t dims[4] = {(uint64_t)Cin, (uint64_t)Win, (uint64_t)Hin, (uint64_t)B};
     uint64_t str[3] = {(uint64_t)Cin * 2, (uint64_t)Win * Cin * 2, (uint64_t)Hin * Win * Cin * 2};
-    uint32_t box[4] = {kBK, (uint32_t)(W * stride), (uint32_t)(BH * stride), (uint32_t)BB};
+    // (stride 2 at a 128-wide tile: a 256-element box with element stride 2, the largest box TMA takes)
+    uint32_t box[4] = {kBK, (uint32_t)((W < 128 ? W : 128) * stride), (uint32_t)(BH * stride), (uint32_t)BB};
     uint32_t es[4] = {1, (uint32_t)stride, (uint32_t)stride, 1};
     if (int e = e4t_tmap_encode(&mA, x, 4, dims, str, box, 2, 128, stride == 1 ? nullptr : es)) return e;
   }
@@ -726,7 +742,17 @@ static int conv3x3_impl(const void* x, const void* w, void* out, int B, int Hin,
 extern "C" int e4t_conv3x3_bf16(const void* x, const void* w, void* out, int B, int H, int W, int Cin, int Cout,
                                 int out_mode, const float* bias, const float* rowgroup, const void* residual,
                                 int force_bn, void* stream_) {
-  return conv3x3_impl(x, w, out, B, H, W, Cin, Cout, 1, out_mode, bias, rowgroup, residual, force_bn,
+  return conv3x3_impl(x, w, out, B, H, W, Cin, Cout, 1, 1, out_mode, bias, rowgroup, residual, force_bn,
+                      (cudaStream_t)stream_);
+}
+
+// General forward 3x3 convolution (bf16 output): stride 1 or 2, top/left padding 1 or 0 (0 with stride 2 only), bias
+// and residual in the epilogue; output widths that divide 128 or are multiples of 128.  x [B][H][W][Cin] ->
+// out [B][H/stride][W/stride][Cout].
+extern "C" int e4t_conv3x3_ex(const void* x, const void* w, void* out, int B, int H, int W, int Cin, int Cout,
+                              int stride, int pad, const float* bias, const void* residual, int force_bn,
+                              void* stream_) {
+  return conv3x3_impl(x, w, out, B, H, W, Cin, Cout, stride, pad, 0, bias, nullptr, residual, force_bn,
                       (cudaStream_t)stream_);
 }
 
@@ -734,7 +760,7 @@ extern "C" int e4t_conv3x3_bf16(const void* x, const void* w, void* out, int B, 
 // out [B][H/2][W/2][Cout].
 extern "C" int e4t_conv3x3_s2_bf16(const void* x, const void* w, void* out, int B, int H, int W, int Cin, int Cout,
                                    const float* bias, int force_bn, void* stream_) {
-  return conv3x3_impl(x, w, out, B, H, W, Cin, Cout, 2, 0, bias, nullptr, nullptr, force_bn, (cudaStream_t)stream_);
+  return conv3x3_impl(x, w, out, B, H, W, Cin, Cout, 2, 1, 0, bias, nullptr, nullptr, force_bn, (cudaStream_t)stream_);
 }
 
 // 3x3 / stride 1 / pad 1 weight gradient: dw9[tap][co][ci] += sum_{b,y,x} dy[b][y][x][co] * x[b][y+ky-1][x+kx-1][ci]

@@ -8,6 +8,13 @@ import torch.nn.functional as F
 from torch import nn
 
 from e4t_b200 import functional as FN
+from e4t_b200 import ops
+
+
+def f32(p):
+    """fp32 view of a bias / norm parameter: the parameter itself when fp32, else a cached fp32 copy (a model cast with
+    .to(dtype=bf16/fp16), e.g. the frozen VAE at pretrain_e4t.py:423)."""
+    return p if p is None or p.dtype == torch.float32 else FN.prepared(p, "f32", lambda t: t.float().contiguous())
 
 
 def conv_w9(conv):
@@ -23,7 +30,7 @@ def conv_w9_dgrad(conv):
 
 
 def conv3x3(conv, x, rowgroup=None, residual=None):
-    return FN.Conv3x3Fn.apply(x, conv_w9(conv), conv_w9_dgrad(conv), conv.bias, rowgroup, residual, conv.weight)
+    return FN.Conv3x3Fn.apply(x, conv_w9(conv), conv_w9_dgrad(conv), f32(conv.bias), rowgroup, residual, conv.weight)
 
 
 class Upsample2D(nn.Module):
@@ -50,8 +57,8 @@ class Upsample2D(nn.Module):
 class Downsample2D(nn.Module):
     def __init__(self, channels, use_conv=False, out_channels=None, padding=1, name="conv"):
         super().__init__()
-        if not use_conv or padding != 1:
-            raise NotImplementedError("SD-v1.x uses 3x3 stride-2 pad-1 conv downsampling only")
+        if not use_conv or padding not in (0, 1):
+            raise NotImplementedError("SD-v1.x uses 3x3 stride-2 conv downsampling with padding 1 (UNet) or 0 (VAE)")
         self.channels = channels
         self.out_channels = out_channels or channels
         self.padding = padding
@@ -65,6 +72,12 @@ class Downsample2D(nn.Module):
     def forward(self, hidden_states):
         # stride-2 convolution computed directly at the output resolution (SURVEY.md §8 a-9)
         c = self.conv
+        if self.padding == 0:
+            # the VAE encoder's F.pad(x, (0,1,0,1)) + pad-0 conv (frozen VAE, forward only); the bottom/right zeros are
+            # the kernel's out-of-bounds fill
+            if torch.is_grad_enabled() and (c.weight.requires_grad or hidden_states.requires_grad):
+                raise NotImplementedError("Downsample2D(padding=0) is forward-only (the VAE is frozen)")
+            return ops.conv3x3_ex(FN._c(hidden_states), conv_w9(c), stride=2, pad=0, bias=f32(c.bias))
         return FN.Conv3x3S2Fn.apply(hidden_states, conv_w9(c), conv_w9_dgrad(c), c.bias, c.weight)
 
 
@@ -110,13 +123,13 @@ class ResnetBlock2D(nn.Module):
             raise NotImplementedError("output_scale_factor != 1")
         x = input_tensor
         n1, n2 = self.norm1, self.norm2
-        h = FN.GroupNormFn.apply(x, n1.weight, n1.bias, n1.num_groups, n1.eps, True)
+        h = FN.GroupNormFn.apply(x, f32(n1.weight), f32(n1.bias), n1.num_groups, n1.eps, True)
         h = conv3x3(self.conv1, h, rowgroup=self.temb_row(temb))
-        h = FN.GroupNormFn.apply(h, n2.weight, n2.bias, n2.num_groups, n2.eps, True)
+        h = FN.GroupNormFn.apply(h, f32(n2.weight), f32(n2.bias), n2.num_groups, n2.eps, True)
         if self.conv_shortcut is not None:
             B, H, W, C = x.shape
             w = FN.prepared(self.conv_shortcut.weight, "bf16_1x1",
                             lambda t: t.reshape(t.shape[0], t.shape[1]).to(torch.bfloat16).contiguous())
-            x = FN.LinearFn.apply(x.view(B, H * W, C), w, self.conv_shortcut.bias, None,
+            x = FN.LinearFn.apply(x.view(B, H * W, C), w, f32(self.conv_shortcut.bias), None,
                                   self.conv_shortcut.weight).view(B, H, W, -1)
         return conv3x3(self.conv2, h, residual=x)

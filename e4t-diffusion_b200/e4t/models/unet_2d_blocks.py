@@ -1,10 +1,12 @@
 """UNet blocks used by SD-v1.x — mirror of e4t/models/unet_2d_blocks.py (vendored diffusers 0.14.0):
 get_down_block/get_up_block (31-372), UNetMidBlock2DCrossAttn (454-551), CrossAttnDownBlock2D (727-855),
-DownBlock2D (858-934), CrossAttnUpBlock2D (1697-1827), UpBlock2D (1830-1901).
+DownBlock2D (858-934), CrossAttnUpBlock2D (1697-1827), UpBlock2D (1830-1901), and the VAE's UNetMidBlock2D
+(375-451), DownEncoderBlock2D (937-994), UpDecoderBlock2D (1904-1955).
 Activations are channels-last (B,H,W,C) bf16; the skip concat is along the last dim."""
 import torch
 from torch import nn
 
+from e4t.models.attention import AttentionBlock
 from e4t.models.resnet import Downsample2D, ResnetBlock2D, Upsample2D
 from e4t.models.transformer_2d import Transformer2DModel
 
@@ -31,6 +33,11 @@ def get_down_block(down_block_type, num_layers, in_channels, out_channels, temb_
                                     use_linear_projection=use_linear_projection,
                                     only_cross_attention=only_cross_attention, upcast_attention=upcast_attention,
                                     resnet_time_scale_shift=resnet_time_scale_shift)
+    if down_block_type == "DownEncoderBlock2D":
+        return DownEncoderBlock2D(num_layers=num_layers, in_channels=in_channels, out_channels=out_channels,
+                                  add_downsample=add_downsample, resnet_eps=resnet_eps, resnet_act_fn=resnet_act_fn,
+                                  resnet_groups=resnet_groups, downsample_padding=downsample_padding,
+                                  resnet_time_scale_shift=resnet_time_scale_shift)
     raise ValueError(f"{down_block_type} is not part of the SD-v1.x E4T path (SURVEY.md §2 #5)")
 
 
@@ -56,6 +63,10 @@ def get_up_block(up_block_type, num_layers, in_channels, out_channels, prev_outp
                                   use_linear_projection=use_linear_projection,
                                   only_cross_attention=only_cross_attention, upcast_attention=upcast_attention,
                                   resnet_time_scale_shift=resnet_time_scale_shift)
+    if up_block_type == "UpDecoderBlock2D":
+        return UpDecoderBlock2D(num_layers=num_layers, in_channels=in_channels, out_channels=out_channels,
+                                add_upsample=add_upsample, resnet_eps=resnet_eps, resnet_act_fn=resnet_act_fn,
+                                resnet_groups=resnet_groups, resnet_time_scale_shift=resnet_time_scale_shift)
     raise ValueError(f"{up_block_type} is not part of the SD-v1.x E4T path (SURVEY.md §2 #5)")
 
 
@@ -238,4 +249,76 @@ class UpBlock2D(nn.Module):
         if self.upsamplers is not None:
             for upsampler in self.upsamplers:
                 hidden_states = upsampler(hidden_states, upsample_size)
+        return hidden_states
+
+
+class UNetMidBlock2D(nn.Module):
+    """The VAE mid-block: resnet, then (AttentionBlock, resnet) x num_layers; no time embedding in the VAE."""
+
+    def __init__(self, in_channels, temb_channels, dropout=0.0, num_layers=1, resnet_eps=1e-6,
+                 resnet_time_scale_shift="default", resnet_act_fn="swish", resnet_groups=32, resnet_pre_norm=True,
+                 add_attention=True, attn_num_head_channels=1, output_scale_factor=1.0):
+        super().__init__()
+        resnet_groups = resnet_groups if resnet_groups is not None else min(in_channels // 4, 32)
+        self.add_attention = add_attention
+        mk = lambda: _resnet(in_channels, in_channels, temb_channels, resnet_eps, resnet_groups, dropout,
+                             resnet_act_fn, resnet_time_scale_shift, output_scale_factor, resnet_pre_norm)
+        resnets = [mk()]
+        attentions = []
+        for _ in range(num_layers):
+            attentions.append(AttentionBlock(in_channels, num_head_channels=attn_num_head_channels,
+                                             rescale_output_factor=output_scale_factor, eps=resnet_eps,
+                                             norm_num_groups=resnet_groups) if add_attention else None)
+            resnets.append(mk())
+        self.attentions = nn.ModuleList(attentions)
+        self.resnets = nn.ModuleList(resnets)
+
+    def forward(self, hidden_states, temb=None):
+        hidden_states = self.resnets[0](hidden_states, temb)
+        for attn, resnet in zip(self.attentions, self.resnets[1:]):
+            if attn is not None:
+                hidden_states = attn(hidden_states)
+            hidden_states = resnet(hidden_states, temb)
+        return hidden_states
+
+
+class DownEncoderBlock2D(nn.Module):
+    def __init__(self, in_channels, out_channels, dropout=0.0, num_layers=1, resnet_eps=1e-6,
+                 resnet_time_scale_shift="default", resnet_act_fn="swish", resnet_groups=32, resnet_pre_norm=True,
+                 output_scale_factor=1.0, add_downsample=True, downsample_padding=1):
+        super().__init__()
+        self.resnets = nn.ModuleList([
+            _resnet(in_channels if i == 0 else out_channels, out_channels, None, resnet_eps, resnet_groups, dropout,
+                    resnet_act_fn, resnet_time_scale_shift, output_scale_factor, resnet_pre_norm)
+            for i in range(num_layers)])
+        self.downsamplers = nn.ModuleList([Downsample2D(out_channels, use_conv=True, out_channels=out_channels,
+                                                        padding=downsample_padding, name="op")]) if add_downsample else None
+
+    def forward(self, hidden_states):
+        for resnet in self.resnets:
+            hidden_states = resnet(hidden_states, temb=None)
+        if self.downsamplers is not None:
+            for downsampler in self.downsamplers:
+                hidden_states = downsampler(hidden_states)
+        return hidden_states
+
+
+class UpDecoderBlock2D(nn.Module):
+    def __init__(self, in_channels, out_channels, dropout=0.0, num_layers=1, resnet_eps=1e-6,
+                 resnet_time_scale_shift="default", resnet_act_fn="swish", resnet_groups=32, resnet_pre_norm=True,
+                 output_scale_factor=1.0, add_upsample=True):
+        super().__init__()
+        self.resnets = nn.ModuleList([
+            _resnet(in_channels if i == 0 else out_channels, out_channels, None, resnet_eps, resnet_groups, dropout,
+                    resnet_act_fn, resnet_time_scale_shift, output_scale_factor, resnet_pre_norm)
+            for i in range(num_layers)])
+        self.upsamplers = nn.ModuleList([Upsample2D(out_channels, use_conv=True, out_channels=out_channels)]) \
+            if add_upsample else None
+
+    def forward(self, hidden_states):
+        for resnet in self.resnets:
+            hidden_states = resnet(hidden_states, temb=None)
+        if self.upsamplers is not None:
+            for upsampler in self.upsamplers:
+                hidden_states = upsampler(hidden_states)
         return hidden_states

@@ -15,8 +15,9 @@ instead of once per step (SURVEY.md §8 f-2).
 
 diffusers is not a dependency: the SD-v1.x DDIM scheduler (scaled-linear betas, steps_offset 1, no sample clipping,
 eta) is `DDIMScheduler` below; any object with set_timesteps / scale_model_input / step(...).prev_sample works.
-VAE decoding is outside SURVEY.md §8: with `vae=None` the pipeline returns latents (`output_type="latent"`); a
-user-supplied `vae` with `.decode(z).sample` is called as the reference does (decode_latents)."""
+With `vae=None` the pipeline returns latents (`output_type="latent"`); with a VAE attached (e.g.
+e4t.models.autoencoder_kl.AutoencoderKL, decoded on the sm_100a kernels) `vae.decode(z).sample` is called as the
+reference does (decode_latents)."""
 from dataclasses import dataclass
 from typing import List, Optional, Union
 
@@ -110,7 +111,8 @@ class StableDiffusionE4TPipeline:
         with torch.no_grad():
             self.class_embed = text_encoder.get_input_embeddings()(ids.to(text_encoder.device))      # :60
         self.domain_embed_scale = e4t_config.domain_embed_scale
-        self.vae_scale_factor = 8
+        # diffusers: 2 ** (len(vae.config.block_out_channels) - 1); 8 (the SD-v1.x VAE) when no VAE is attached
+        self.vae_scale_factor = 2 ** (len(vae.config.block_out_channels) - 1) if vae is not None else 8
 
     @property
     def _execution_device(self):
@@ -144,7 +146,7 @@ class StableDiffusionE4TPipeline:
 
     def decode_latents(self, latents):
         if self.vae is None:
-            raise NotImplementedError("no VAE attached: use output_type='latent' (VAE decode is outside SURVEY.md §8)")
+            raise NotImplementedError("no VAE attached: pass vae=AutoencoderKL(...) or use output_type='latent'")
         image = self.vae.decode(latents / 0.18215).sample
         return (image / 2 + 0.5).clamp(0, 1).cpu().permute(0, 2, 3, 1).float().numpy()
 

@@ -5,7 +5,8 @@ reference gets from accelerate/torch.optim rebuilt B200-first:
                     gradient arena; the optimiser is a single fused sm_100a kernel over the arena and the
                     data-parallel gradient exchange is ONE NCCL all-reduce of the gradient arena
                     (reference: DDP buckets over every requires_grad parameter, ≈4.9 GB; here 1.5 GB).
-  * PretrainStep  — the loop body given explicit (pixel_values, latents, noise, timesteps, input_ids).
+  * PretrainStep  — the loop body given explicit (pixel_values, latents, noise, timesteps, input_ids); with a VAE
+                    attached, `latents` may be replaced by `latent_eps` and are then encoded on the device.
 """
 import os
 
@@ -166,8 +167,12 @@ class PretrainStep:
     def __init__(self, unet, e4t_encoder, text_encoder, placeholder_token_id, class_token_id, lr=1.6e-5,
                  betas=(0.9, 0.999), weight_decay=1e-2, eps=1e-8, domain_embed_scale=0.1, reg_lambda=0.01,
                  bos_id=49406, eos_id=49407, weight_dtype=torch.bfloat16, optimizer=True, tune_unet=False,
-                 max_grad_norm=None):
+                 max_grad_norm=None, vae=None):
         self.unet, self.enc, self.text = unet, e4t_encoder, text_encoder
+        # frozen AutoencoderKL (pretrain_e4t.py:262): batches without `latents` are encoded from their pixel_values
+        self.vae = vae
+        if vae is not None:
+            vae.requires_grad_(False)
         self.placeholder_token_id = placeholder_token_id
         self.domain_embed_scale, self.reg_lambda = domain_embed_scale, reg_lambda
         self.weight_dtype = weight_dtype
@@ -222,8 +227,17 @@ class PretrainStep:
         return [row.index(self.placeholder_token_id) for row in input_ids.cpu().tolist()]
 
     def forward_loss(self, batch):
-        pixel_values, latents, noise = batch["pixel_values"], batch["latents"], batch["noise"]
+        pixel_values, noise = batch["pixel_values"], batch["noise"]
         timesteps, input_ids = batch["timesteps"], batch["input_ids"]
+        latents = batch.get("latents")
+        if latents is None and self.vae is not None:
+            # pretrain_e4t.py:597-599 with the sample's ε taken from the batch (like `noise`), so that the encode is
+            # part of a captured step: latent_dist.sample() == mean + std * ε
+            with torch.no_grad():
+                d = self.vae.encode(pixel_values).latent_dist
+                latents = (d.mean + d.std * batch["latent_eps"]) * self.vae.config.scaling_factor
+        elif latents is None:
+            raise KeyError("batch has no 'latents' and no VAE is attached to encode its pixel_values")
         B = latents.shape[0]
         emb = self.text.get_input_embeddings()
         with torch.no_grad():

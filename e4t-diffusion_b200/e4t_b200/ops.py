@@ -97,6 +97,33 @@ def conv3x3_s2(x, w9, *, bias=None, force_bn=0):
     return out
 
 
+def conv3x3_ex(x, w9, *, stride=1, pad=1, bias=None, residual=None, force_bn=0):
+    """3x3 convolution on NHWC bf16 with stride 1/2 and top/left padding 1, or 0 with stride 2 (the VAE's
+    F.pad(x, (0,1,0,1)) downsample): (B,H,W,Cin) -> (B,H/stride,W/stride,Cout) bf16."""
+    assert x.dtype == BF16 and w9.dtype == BF16 and x.is_contiguous() and w9.is_contiguous()
+    Bn, H, W, Cin = x.shape
+    Cout = w9.shape[1]
+    assert w9.shape == (9, Cout, Cin)
+    out = torch.empty((Bn, H // stride, W // stride, Cout), device=x.device, dtype=BF16)
+    if residual is not None:
+        assert residual.dtype == BF16 and residual.is_contiguous() and residual.shape == out.shape
+    _lib.call("e4t_conv3x3_ex", ptr(x), ptr(w9), ptr(out), c_int(Bn), c_int(H), c_int(W), c_int(Cin), c_int(Cout),
+              c_int(stride), c_int(pad), ptr(bias), ptr(residual), c_int(force_bn), stream())
+    return out
+
+
+def softmax_rows(S, out=None):
+    """Row softmax of an fp32 matrix (.., M) (last dim contiguous, rows evenly strided) -> bf16 of the same shape."""
+    assert S.dtype == F32 and S.stride(-1) == 1
+    M = S.shape[-1]
+    S2 = S.reshape(-1, M) if S.dim() != 2 else S
+    if out is None:
+        out = torch.empty(S.shape, device=S.device, dtype=BF16)
+    assert out.is_contiguous() and S2.stride(0) == M
+    _lib.call("e4t_softmax_rows", ptr(S2), ptr(out), c_ll(S2.shape[0]), c_int(M), c_ll(M), stream())
+    return out
+
+
 # ----------------------------------------------------------------------------------------------
 # normalisation
 # ----------------------------------------------------------------------------------------------
@@ -208,6 +235,17 @@ def conv_in_fwd(x, w, bias):
     y = torch.empty((Bn, H, W, Cout), device=x.device, dtype=BF16)
     _lib.call("e4t_conv_in_fwd", ptr(x), ptr(w), ptr(bias), ptr(y), c_int(Bn), c_int(Cin), c_int(H), c_int(W),
               c_int(Cout), stream())
+    return y
+
+
+def pointwise_nchw(x, w, bias):
+    """1x1 convolution on NCHW fp32 (B,Cin,H,W) -> (B,Cout,H,W); w fp32 (Cout,Cin)."""
+    assert x.dtype == F32 and x.is_contiguous() and w.dtype == F32 and w.is_contiguous()
+    Bn, Cin, H, W = x.shape
+    Cout = w.shape[0]
+    y = torch.empty((Bn, Cout, H, W), device=x.device, dtype=F32)
+    _lib.call("e4t_pointwise_nchw", ptr(x), ptr(w), ptr(bias), ptr(y), c_int(Bn), c_int(Cin), c_int(Cout),
+              c_ll(H * W), stream())
     return y
 
 

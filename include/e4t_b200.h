@@ -49,6 +49,13 @@ int e4t_conv3x3_bf16(const void* x, const void* w, void* out, int B, int H, int 
  * out [B][H/2][W/2][Cout]. */
 int e4t_conv3x3_s2_bf16(const void* x, const void* w, void* out, int B, int H, int W, int Cin, int Cout,
                         const float* bias, int force_bn, void* stream);
+/* General forward 3x3 convolution for the VAE (diffusers AutoencoderKL Encoder/Decoder): stride 1 or 2; top/left
+ * padding `pad` 1, or 0 with stride 2 (Downsample2D(padding=0) == F.pad(x, (0,1,0,1)) + pad-0 conv; the bottom/right
+ * zeros come from the TMA out-of-bounds fill).  Output width W/stride divides 128 or is a multiple of 128 (wide images:
+ * one M tile = 128 pixels of one row).  x [B][H][W][Cin] -> out [B][H/stride][W/stride][Cout] bf16; bias fp32 [Cout];
+ * residual bf16 like out or null. */
+int e4t_conv3x3_ex(const void* x, const void* w, void* out, int B, int H, int W, int Cin, int Cout, int stride, int pad,
+                   const float* bias, const void* residual, int force_bn, void* stream);
 /* Weight gradient of the 3x3 / stride 1 / pad 1 convolution: dw9[tap][co][ci] += sum dy[b][y][x][co] * x[b][y+ky-1][x+kx-1][ci]
  * (fp32 atomic accumulation; implicit GEMM with 9 taps as the batch dimension, split-K over pixels).  Replaces autograd's
  * conv2d weight gradient when the base UNet is trainable (tuning_e4t.py:139-146; every requires_grad parameter under
@@ -97,6 +104,11 @@ int e4t_attn_small_bwd(const void* Q, const void* K, const void* V, const void* 
                        long long lddo, long long do_bs, long long lddq, long long dq_bs, long long lddk, long long dk_bs,
                        long long lddv, long long dv_bs, float scale, int causal, void* stream);
 
+/* Row softmax P[r][:M] = softmax(S[r][:M]) (fp32 in, bf16 out, row stride ld for both; M, ld % 4 == 0): the middle of
+ * the three launches of the VAE mid-block AttentionBlock (diffusers attention.py AttentionBlock.forward),
+ * S = alpha Q K^T and O = P V being e4t_gemm_bf16 calls.  No length limit on M. */
+int e4t_softmax_rows(const float* S, void* P, long long rows, int M, long long ld, void* stream);
+
 /* ---- normalisation ------------------------------------------------------------------------------------------- */
 /* GroupNorm (+ optional fused SiLU).  Replaces nn.GroupNorm + F.silu in diffusers ResnetBlock2D, Transformer2DModel
  * .norm (transformer_2d.py:149,253) and conv_norm_out/conv_act (unet_2d_condition.py:554-556).
@@ -142,6 +154,10 @@ int e4t_resample2x(const void* x, void* y, int B, int H, int W, int C, int mode,
 /* UNet conv_in (unet_2d_condition.py:481): NCHW fp32 -> NHWC bf16; w fp32 [Cout][Cin][3][3]. */
 int e4t_conv_in_fwd(const float* x, const float* w, const float* bias, void* y, int B, int Cin, int H, int W,
                     int Cout, void* stream);
+/* 1x1 convolution on NCHW fp32 (Cin, Cout <= 8): the VAE's post_quant_conv on the latents before Decoder.conv_in.
+ * w fp32 [Cout][Cin]; bias fp32 [Cout] or null. */
+int e4t_pointwise_nchw(const float* x, const float* w, const float* bias, float* y, int B, int Cin, int Cout,
+                       long long HW, void* stream);
 /* UNet conv_out (unet_2d_condition.py:557): NHWC bf16 -> NCHW fp32, and its input gradient. */
 int e4t_conv_out_fwd(const void* x, const float* w, const float* bias, float* y, int B, int H, int W, int C, int Cout,
                      void* stream);
