@@ -37,6 +37,7 @@ struct GemmArgs {
   int debug;      // E4T_GEMM_DEBUG probes: 1 skip epilogue body, 4 skip output staging, 8 no TMA loads, 16 no MMAs
   int tma_store;  // bf16 output through smem staging + TMA store (coalesced, asynchronous)
   int epi_plain;  // default on (E4T_GEMM_EPI_PLAIN=0 disables): separate slab loop for outputs without alpha/bias/rowgroup/residual
+  int epi_vec;    // the per-thread epilogue's 16-byte accesses (output, residual, row-group rows) are aligned; else scalar
 };
 
 static constexpr int kBM = 128;
@@ -427,7 +428,7 @@ e4t_gemm_kernel(const __grid_constant__ CUtensorMap mapA, const __grid_constant_
           float f[8];
 #pragma unroll
           for (int j = 0; j < 8; ++j) f[j] = __uint_as_float(v[q * 8 + j]) * g.alpha;
-          const bool full8 = (n + 8 <= g.N);
+          const bool full8 = g.epi_vec && (n + 8 <= g.N);
           if (full8) {
             if (g.bias) {
               const float4 b0 = *reinterpret_cast<const float4*>(g.bias + n);
@@ -581,8 +582,20 @@ static int launch_gemm(const CUtensorMap& mA, const CUtensorMap& mB, GemmArgs& g
     const char* e = getenv("E4T_GEMM_TMA_STORE");
     use_tma_store = (e && e[0] == '0') ? 0 : 1;
   }
+  // Epilogue alignment (include/e4t_b200.h).  Bias and row-group rows are read as float4 at multiples of 8 columns on
+  // every path, so their base pointers must be 16-byte aligned.  The output, residual and row-group row strides only
+  // choose the path: every 16-byte access of the per-thread loop is aligned (epi_vec), or that loop goes scalar.
+  E4T_CHECK(((uintptr_t)g.bias % 16) == 0 && ((uintptr_t)g.rowgroup % 16) == 0,
+            "e4t_gemm: bias and rowgroup must be 16-byte aligned");
+  const int out_el = g.out_mode == 0 ? 8 : 4;  // output elements per 16 bytes
+  const bool out_vec = g.out_mode == 2 || (((uintptr_t)g.out % 16) == 0 && (g.ldo % out_el) == 0 &&
+                                           (g.batch == 1 || (g.out_bstride % out_el) == 0));
+  const bool res_vec = !g.residual || (((uintptr_t)g.residual % 16) == 0 && (g.ldr % 8) == 0 &&
+                                       (g.batch == 1 || (g.res_bstride % 8) == 0));
+  const bool rg_vec = !g.rowgroup || (g.N % 4) == 0;
+  g.epi_vec = out_vec && res_vec && rg_vec;
   if (use_tma_store && g.out_mode == 0 && (g.N % 8) == 0 && (g.ldo % 8) == 0 && ((uintptr_t)g.out % 16) == 0 &&
-      (g.batch == 1 || (g.out_bstride % 8) == 0)) {
+      (g.batch == 1 || (g.out_bstride % 8) == 0) && res_vec) {
     uint64_t dims[3] = {(uint64_t)g.N, (uint64_t)g.M, (uint64_t)g.batch};
     uint64_t str[2] = {(uint64_t)g.ldo * 2, (uint64_t)(g.batch > 1 ? g.out_bstride : (long long)g.M * g.ldo) * 2};
     uint32_t box[3] = {32, kBM, 1};
@@ -635,6 +648,8 @@ extern "C" int e4t_gemm_bf16(const void* A, const void* B, void* out, int M, int
   E4T_CHECK(g.BN >= 32 && g.BN <= 256 && (g.BN % (b_mn ? 64 : 32)) == 0, "e4t_gemm_bf16: bad BN %d", g.BN);
   g.n_tiles = cdiv(N, g.BN);
   E4T_CHECK(g.splits == 1 || out_mode == 2, "e4t_gemm_bf16: split-K requires atomic fp32 output");
+  // every split would add them again
+  E4T_CHECK(g.splits == 1 || (!bias && !rowgroup && !residual), "e4t_gemm_bf16: split-K takes no bias/rowgroup/residual");
   g.out = out; g.out_mode = out_mode; g.ldo = ldo; g.out_bstride = out_bstride;
   g.bias = bias; g.rowgroup = rowgroup; g.rows_per_group = rows_per_group > 0 ? rows_per_group : 1;
   g.residual = (const bf16*)residual; g.ldr = ldr; g.res_bstride = res_bstride;
@@ -716,6 +731,7 @@ static int conv3x3_impl(const void* x, const void* w, void* out, int B, int Hin,
   g.kchunks = 9 * g.cin_chunks;
   g.kper = g.kchunks; g.splits = 1;
   g.BN = pick_bn(Cout, g.m_tiles, false, force_bn, g.kchunks, residual != nullptr, false);
+  E4T_CHECK(g.BN >= 32 && g.BN <= 256 && (g.BN % 32) == 0, "e4t_conv3x3: bad BN %d", g.BN);
   g.n_tiles = cdiv(Cout, g.BN);
   g.out = out; g.out_mode = out_mode; g.ldo = Cout; g.out_bstride = 0;
   g.bias = bias; g.rowgroup = rowgroup; g.rows_per_group = img;

@@ -39,24 +39,33 @@ __device__ __forceinline__ void unpack8(const uint4& u, float* f) {
 __device__ __forceinline__ uint4 pack8(const float* f) {
   return make_uint4(pack_bf16(f[0], f[1]), pack_bf16(f[2], f[3]), pack_bf16(f[4], f[5]), pack_bf16(f[6], f[7]));
 }
+// The forward sums of group g of image b are taken about a pivot, the group's first element p = x[b][0][g * cpg]:
+// (Σ(x - p), Σ(x - p)²).  Σx² / n - mean² would lose the variance to cancellation, with a relative error that grows as
+// (mean / std)²; about a sample of the group the two terms are of the order of the variance itself.
+__device__ __forceinline__ float gn_pivot(const bf16* __restrict__ x, int b, int g, int HW, int C, int cpg) {
+  return __bfloat162float(x[(long)b * HW * C + g * cpg]);
+}
+__device__ __forceinline__ void gn_mean_rstd(const float* __restrict__ stats, const bf16* __restrict__ x, int b, int g,
+                                             int HW, int C, int G, float inv_n, float eps, float& mean, float& rstd) {
+  const float d = stats[((long)b * G + g) * 2] * inv_n, ss = stats[((long)b * G + g) * 2 + 1] * inv_n;
+  mean = gn_pivot(x, b, g, HW, C, C / G) + d;
+  rstd = rsqrtf(fmaxf(ss - d * d, 0.f) + eps);
+}
 // per-channel (mean, rstd, gamma, beta) of this thread's 8 channels, from the forward sums
-__device__ __forceinline__ void gn_thread_chan(GNChan* ch, const float* __restrict__ stats,
+__device__ __forceinline__ void gn_thread_chan(GNChan* ch, const float* __restrict__ stats, const bf16* __restrict__ x,
                                                const float* __restrict__ gamma, const float* __restrict__ beta, int b,
-                                               int c0, int C, int G, float inv_n, float eps) {
+                                               int c0, int HW, int C, int G, float inv_n, float eps) {
   const int cpg = C / G;
 #pragma unroll
   for (int j = 0; j < 8; ++j) {
-    const int g = (c0 + j) / cpg;
-    const float s = stats[((long)b * G + g) * 2], ss = stats[((long)b * G + g) * 2 + 1];
-    const float mean = s * inv_n;
-    ch[j].mean = mean;
-    ch[j].rstd = rsqrtf(fmaxf(ss * inv_n - mean * mean, 0.f) + eps);
+    gn_mean_rstd(stats, x, b, (c0 + j) / cpg, HW, C, G, inv_n, eps, ch[j].mean, ch[j].rstd);
     ch[j].gamma = gamma[c0 + j];
     ch[j].beta = beta[c0 + j];
   }
 }
 
-// sums[b][g] += (Σ a, Σ b) over this CTA's rows.  MODE 0: (x, x²).  MODE 1: (dxhat, dxhat·xhat).
+// sums[b][g] += (Σ a, Σ b) over this CTA's rows.  MODE 0: (x - p, (x - p)²), p = the group's pivot (gn_pivot).
+// MODE 1: (dxhat, dxhat·xhat).
 template <int MODE>
 __global__ void __launch_bounds__(kGNMaxThreads)
 gn_stats_kernel(const bf16* __restrict__ x, const bf16* __restrict__ dy, const float* __restrict__ fstats,
@@ -71,11 +80,15 @@ gn_stats_kernel(const bf16* __restrict__ x, const bf16* __restrict__ dy, const f
   const int r0 = blockIdx.x * rows_per_cta;
   const int r1 = min(HW, r0 + rows_per_cta);
   GNChan ch[8];
-  if (MODE == 1) gn_thread_chan(ch, fstats, gamma, beta, b, c0, C, G, 1.f / ((float)HW * (float)(C / G)), eps);
+  float piv[8];
+  if (MODE == 1) gn_thread_chan(ch, fstats, x, gamma, beta, b, c0, HW, C, G, 1.f / ((float)HW * (float)(C / G)), eps);
   __syncthreads();
   float a0[8], a1[8];
 #pragma unroll
-  for (int j = 0; j < 8; ++j) a0[j] = a1[j] = 0.f;
+  for (int j = 0; j < 8; ++j) {
+    a0[j] = a1[j] = 0.f;
+    if (MODE == 0) piv[j] = gn_pivot(x, b, (c0 + j) / (C / G), HW, C, C / G);
+  }
   const bf16* xb = x + ((long)b * HW) * C + c0;
   const bf16* db = MODE == 1 ? dy + ((long)b * HW) * C + c0 : nullptr;
 #pragma unroll 4
@@ -85,8 +98,9 @@ gn_stats_kernel(const bf16* __restrict__ x, const bf16* __restrict__ dy, const f
     if (MODE == 0) {
 #pragma unroll
       for (int j = 0; j < 8; ++j) {
-        a0[j] += xv[j];
-        a1[j] += xv[j] * xv[j];
+        const float d = xv[j] - piv[j];
+        a0[j] += d;
+        a1[j] += d * d;
       }
     } else {
       float dv[8];
@@ -130,7 +144,7 @@ gn_apply_kernel(const bf16* __restrict__ x, const bf16* __restrict__ dy, const f
   const int cv = threadIdx.x % vpr, rl = threadIdx.x / vpr, rstep = blockDim.x / vpr;
   const int c0 = cv * 8;
   GNChan ch[8];
-  gn_thread_chan(ch, fstats, gamma, beta, b, c0, C, G, inv_n, eps);
+  gn_thread_chan(ch, fstats, x, gamma, beta, b, c0, HW, C, G, inv_n, eps);
   float scale[8], shift[8], m1[8], m2[8];
   const int cpg = C / G;
 #pragma unroll
@@ -207,7 +221,7 @@ static int gn_block(int C) {
   return vpr * k;
 }
 
-// stats: fp32 [B][G][2] = (sum, sumsq); written by this call.
+// stats: fp32 [B][G][2] = (Σ(x - p), Σ(x - p)²) about the pivot p = x[b][0][g * C / G]; written by this call.
 extern "C" int e4t_groupnorm_fwd(const void* x, const float* gamma, const float* beta, void* y, float* stats, int B,
                                  int HW, int C, int G, float eps, int act_silu, void* stream_) {
   cudaStream_t st = (cudaStream_t)stream_;

@@ -21,7 +21,8 @@ softmax_rows_kernel(const float* __restrict__ S, bf16* __restrict__ P, int M, lo
       sm *= __expf(mx - m4);
       mx = m4;
     }
-    sm += __expf(v.x - mx) + __expf(v.y - mx) + __expf(v.z - mx) + __expf(v.w - mx);
+    // (while every value seen is -inf, exp(-inf - -inf) would make the sum NaN for good)
+    if (mx != -INFINITY) sm += __expf(v.x - mx) + __expf(v.y - mx) + __expf(v.z - mx) + __expf(v.w - mx);
   }
   // merge (max, sum) pairs: warp, then CTA
   float wm = warp_max(mx);

@@ -128,7 +128,8 @@ def softmax_rows(S, out=None):
 # normalisation
 # ----------------------------------------------------------------------------------------------
 def groupnorm_fwd(x, gamma, beta, groups, eps, silu):
-    """x: (B,HW,C) or (B,H,W,C) bf16 NHWC.  Returns (y, stats[B,G,2] = (sum, sumsq))."""
+    """x: (B,HW,C) or (B,H,W,C) bf16 NHWC.  Returns (y, stats[B,G,2] = (sum, sumsq) of x - p), p = each group's first
+    element x[b, 0, g * C // G] (see groupnorm_mean_rstd)."""
     assert x.dtype == BF16 and x.is_contiguous()
     Bn, C = x.shape[0], x.shape[-1]
     HW = x.numel() // (Bn * C)
@@ -455,14 +456,22 @@ def layernorm_param_grad(x, dy, stats, gamma):
     return dg, db
 
 
-def groupnorm_param_grad(x, dy, stats, gamma, beta, groups, eps, silu):
-    """(dgamma, dbeta) fp32 of GroupNorm(+SiLU); stats = the forward's (sum, sum of squares) per (image, group)."""
+def groupnorm_mean_rstd(x, stats, groups, eps):
+    """(mean, rstd) fp32 (B, G) from groupnorm_fwd's stats, which are sums about each group's first element."""
     Bn, C = x.shape[0], x.shape[-1]
     HW = x.numel() // (Bn * C)
     n = float(HW * (C // groups))
-    mean = stats[..., 0] / n
-    var = (stats[..., 1] / n - mean * mean).clamp_min(0.0)
-    rstd = torch.rsqrt(var + eps)
+    pivot = x.reshape(Bn, HW, C)[:, 0, ::C // groups].float()
+    d = stats[..., 0] / n
+    var = (stats[..., 1] / n - d * d).clamp_min(0.0)
+    return pivot + d, torch.rsqrt(var + eps)
+
+
+def groupnorm_param_grad(x, dy, stats, gamma, beta, groups, eps, silu):
+    """(dgamma, dbeta) fp32 of GroupNorm(+SiLU); stats = the forward's per-(image, group) sums."""
+    Bn, C = x.shape[0], x.shape[-1]
+    HW = x.numel() // (Bn * C)
+    mean, rstd = groupnorm_mean_rstd(x, stats, groups, eps)
     mean_c = mean.repeat_interleave(C // groups, dim=1).contiguous()
     rstd_c = rstd.repeat_interleave(C // groups, dim=1).contiguous()
     dg = torch.zeros(C, device=x.device, dtype=F32)

@@ -28,8 +28,19 @@ void e4t_reset_launch_count(void);
  * a_mn / b_mn = 0: operand stored [rows][K] (K contiguous); = 1: stored [K][rows] (rows contiguous).
  * lda/ldb: row stride in elements (multiple of 8); a_bstride/b_bstride: batch stride, 0 = shared across the batch.
  * out_mode 0: bf16 store, 1: fp32 store, 2: fp32 atomic accumulate (required when splits > 1: split-K).
+ * ldo / out_bstride: output row / batch stride in elements; ldr / res_bstride: the same for the bf16 residual.
  * splits: split-K factor; 0 with out_mode 2 = chosen by the library's tile cost model (weight gradients).
- * force_bn: N-tile override for tuning (0 = heuristic). */
+ * force_bn: N-tile override for tuning (0 = heuristic).
+ * Alignment (also for the convolutions below, whose epilogue this is):
+ *   - refused (non-zero return, nothing launched): A or B not 16-byte aligned, lda or ldb not a multiple of 8, bias or
+ *     rowgroup not 16-byte aligned.  The rowgroup's row stride is N.  Also refused: splits > 1 with a bias, rowgroup or
+ *     residual, and a force_bn outside [32, 256] or not a multiple of 32 (of 64 with b_mn).
+ *   - any other pointer, ldo, ldr or batch stride is accepted; it only selects the epilogue.  A bf16 output goes
+ *     through the TMA store when N, ldo (and out_bstride if batch > 1) are multiples of 8, out is 16-byte aligned and
+ *     the residual is vectorisable (below).  Otherwise each thread stores 8 columns per 16-byte access if out is
+ *     16-byte aligned and ldo / out_bstride are multiples of 16 bytes in the output type, the residual is vectorisable
+ *     and (with a rowgroup) N % 4 == 0, and one element at a time if not.  The residual is vectorisable when it is
+ *     16-byte aligned and ldr (and res_bstride if batch > 1) are multiples of 8. */
 int e4t_gemm_bf16(const void* A, const void* B, void* out, int M, int N, int K, int batch, int a_mn, int b_mn,
                   long long lda, long long ldb, long long a_bstride, long long b_bstride, int out_mode,
                   long long ldo, long long out_bstride, const float* bias, const float* rowgroup,
@@ -106,13 +117,16 @@ int e4t_attn_small_bwd(const void* Q, const void* K, const void* V, const void* 
 
 /* Row softmax P[r][:M] = softmax(S[r][:M]) (fp32 in, bf16 out, row stride ld for both; M, ld % 4 == 0): the middle of
  * the three launches of the VAE mid-block AttentionBlock (diffusers attention.py AttentionBlock.forward),
- * S = alpha Q K^T and O = P V being e4t_gemm_bf16 calls.  No length limit on M. */
+ * S = alpha Q K^T and O = P V being e4t_gemm_bf16 calls.  No length limit on M.  Entries may be -inf (masked) as long
+ * as a row keeps one finite entry; P's columns M..ld-1 are not written.  S 16-byte and P 8-byte aligned. */
 int e4t_softmax_rows(const float* S, void* P, long long rows, int M, long long ld, void* stream);
 
 /* ---- normalisation ------------------------------------------------------------------------------------------- */
 /* GroupNorm (+ optional fused SiLU).  Replaces nn.GroupNorm + F.silu in diffusers ResnetBlock2D, Transformer2DModel
  * .norm (transformer_2d.py:149,253) and conv_norm_out/conv_act (unet_2d_condition.py:554-556).
- * x,y [B][HW][C] bf16; stats fp32 [B][G][2] = (sum, sum of squares), written by fwd and consumed by bwd. */
+ * x,y [B][HW][C] bf16; stats fp32 [B][G][2] = (Σ(x - p), Σ(x - p)²) over the group, taken about its first element
+ * p = x[b][0][g * C/G] (mean = p + Σ(x - p)/n, var = Σ(x - p)²/n - (Σ(x - p)/n)², free of the cancellation of
+ * Σx²/n - mean² for groups whose mean is large against their spread); written by fwd and consumed by bwd with the same x. */
 int e4t_groupnorm_fwd(const void* x, const float* gamma, const float* beta, void* y, float* stats, int B, int HW,
                       int C, int G, float eps, int act_silu, void* stream);
 int e4t_groupnorm_bwd(const void* x, const void* dy, const float* gamma, const float* beta, const float* stats,
